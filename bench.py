@@ -6,7 +6,7 @@ each, 50-step PLMS, classifier-free guidance 7.5, alpha schedule [0.8, 0, 0.2], 
 One "step" of the bench contract = one full `sampler.sample(...)` call over one batch (latent out);
 timed region = the sampler only (no CLIP, no VAE), as SURVEY.md section 8d prescribes.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--mis 0.0] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--mis 0.0] [--impl reference] [--dump-outputs DIR]
 
 N > 1: launched under torch.distributed.run, one rank per GPU; rank 0's synthetic weights are
 broadcast once over NCCL, every rank then samples its own batch of prompts (weak scaling, no
@@ -395,7 +395,14 @@ def main():
     ap.add_argument("--dtype", default=None, choices=["fp16", "bf16"],
                     help="16-bit storage type (default: the config's own -- fp16, bf16 for config 4)")
     ap.add_argument("--no-mis-leg", action="store_true", help="skip the extra mis=0.36 leg of config 2")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the float32 latents of the last timed step to DIR/latent.npy (and DIR/mis036_latent.npy "
+                         "for the mis=0.36 leg), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA arm (the reference arm times single forwards, not the sampler)")
     _claim_stdout()
     cfg = CONFIGS[args.config]
     WORKLOAD, BATCH, N_INST, FLAVOR, LATENT = cfg["workload"], cfg["batch"], cfg["n"], cfg["flavor"], cfg["latent"]
@@ -465,6 +472,7 @@ def main():
         parallel.barrier()
         t_dev = parallel.max_over_ranks(ev[0].elapsed_time(ev[1]) * 1e-3, device)
         assert torch.isfinite(out).all()
+        latent = out.float().cpu()  # the last timed step's result, for --dump-outputs
         result_host = torch.empty(shape, dtype=torch.float32).pin_memory()
         torch.cuda.synchronize()
         parallel.barrier()
@@ -481,7 +489,8 @@ def main():
         t_e2e = parallel.max_over_ranks(ev2[0].elapsed_time(ev2[1]) * 1e-3, device)
         images = BATCH * steps * world
         return dict(value=images / t_dev, e2e=images / t_e2e, ms_per_step=t_dev / steps * 1e3, h2d=h2d_bytes,
-                    d2h=result_host.numel() * 4, clocks=clk.summary(), fpc=forwards_per_sample_call(S_STEPS, N_INST, mis))
+                    d2h=result_host.numel() * 4, clocks=clk.summary(), fpc=forwards_per_sample_call(S_STEPS, N_INST, mis),
+                    latent=latent)
 
     peak_tf = peaks.get("bf16_tflops_sustained") or 1400.0
     head = measure(args.mis, args.steps, args.warmup)
@@ -492,6 +501,13 @@ def main():
         mis_leg = measure(MIS_DEFAULT, max(1, min(args.steps, 3)), 1)
     if rank != 0:
         return
+    if args.dump_outputs:
+        # the latents sample() handed back in the last timed step of each leg (rank 0's batch; seeded inputs)
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "latent.npy"), head["latent"].numpy())
+        if mis_leg is not None:
+            np.save(os.path.join(args.dump_outputs, "mis036_latent.npy"), mis_leg["latent"].numpy())
     roof, breakdown, launches_per_fwd = roofline_pass(model, device, peaks)
     value, fpc = head["value"], head["fpc"]
     line = {

@@ -301,6 +301,41 @@ def gen_clip():
     torch.save(out, os.path.join(GOLDEN, "clip_text.pt"))
 
 
+def gen_layout(ref):
+    """tests/golden/reference_layout.json: the import structure of the reference's packages that dropin.install()
+    shadows or keeps as parents (ldm, grounding_input, utils, dataset) -- per file, in order, its module-level
+    imports and the names it defines (class / function / other), no code.  The drop-in test rebuilds a stub tree
+    from it, so that name resolution through the reference's own import graph is checked without the checkout."""
+    import ast
+    layout = {}
+    for top in ("ldm", "grounding_input", "utils", "dataset"):
+        for dirpath, dirnames, files in os.walk(os.path.join(ref.root, top)):
+            dirnames[:] = sorted(d for d in dirnames if d != "__pycache__")
+            for f in sorted(files):
+                if not f.endswith(".py"):
+                    continue
+                path = os.path.join(dirpath, f)
+                stmts = []
+                for s in ast.parse(open(path).read()).body:
+                    if isinstance(s, ast.Import):
+                        stmts += [["import", a.name, a.asname] for a in s.names]
+                    elif isinstance(s, ast.ImportFrom):
+                        stmts.append(["from", s.level, s.module, [[a.name, a.asname] for a in s.names]])
+                    elif isinstance(s, ast.ClassDef):
+                        stmts.append(["class", s.name])
+                    elif isinstance(s, (ast.FunctionDef, ast.AsyncFunctionDef)):
+                        stmts.append(["def", s.name])
+                    elif isinstance(s, (ast.Assign, ast.AnnAssign)):
+                        for t in (s.targets if isinstance(s, ast.Assign) else [s.target]):
+                            names = t.elts if isinstance(t, (ast.Tuple, ast.List)) else [t]
+                            stmts += [["value", n.id] for n in names if isinstance(n, ast.Name)]
+                layout[os.path.relpath(path, ref.root).replace(os.sep, "/")] = stmts
+    with open(os.path.join(GOLDEN, "reference_layout.json"), "w") as fh:  # one statement per line
+        fh.write("{\n" + ",\n".join(json.dumps(path) + ": [\n" + ",\n".join(json.dumps(s) for s in stmts) + "\n]"
+                                     for path, stmts in sorted(layout.items())) + "\n}\n")
+    print(f"  {len(layout)} files")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--threads", type=int, default=os.cpu_count())
@@ -331,6 +366,8 @@ def main():
         print("masked gated self-attention cases"); gen_masked(ref)
     if "vae" in only:
         print("first-stage (VAE) cases"); gen_vae(ref)
+    if "layout" in only:
+        print("reference package layout"); gen_layout(ref)
     if any(o.startswith("unet_extra") or o.startswith("samplers_extra") for o in only):
         print("round-2 unet / sampler cases"); gen_extra(ref, only)
 
