@@ -18,8 +18,6 @@
 #include "common.cuh"
 #include "host.cuh"
 
-#include <stdlib.h>
-
 namespace idiff {
 
 namespace att2 {
@@ -36,14 +34,14 @@ struct AttnKParams {
   int out_ld;
 };
 
-// KV = keys per tile.  64 keeps the footprint of head_dim 80 at 112 KiB of shared memory and 256 TMEM
-// columns, so two CTAs are resident per SM and cover each other's softmax / hand-off latency (what took
-// attention2 from 566 to 414 us); 128 is the one-CTA-per-SM layout (IDIFF_ATT_BKV=128 for A/B runs).
-template <int D, int KV>
+// 64 keys per tile keep the footprint of head_dim 80 at 112 KiB of shared memory and 256 TMEM columns, so two
+// CTAs are resident per SM and cover each other's softmax / hand-off latency (what took attention2 from 566 to
+// 414 us).  128-key tiles, one CTA per SM, measured slower: profiles/README.md round 2, section 7.9.
+template <int D>
 struct AttnCfg {
   static constexpr int ND = (D + 63) / 64;           // 64-wide d chunks (one TMA box each)
   static constexpr int KSTEPS = (D + 15) / 16;       // UMMA k-steps of QK^T (zero padded)
-  static constexpr int BKV = KV;                     // keys per tile
+  static constexpr int BKV = 64;                     // keys per tile
   static constexpr int DV = ND * 64;                 // UMMA N of the PV product
   static constexpr int STAGES = (D <= 64) ? 3 : 2;
   static constexpr int Q_BYTES = ND * BQ * 128;
@@ -59,12 +57,12 @@ struct AttnCfg {
   static constexpr int MIN_CTAS = (SMEM_BYTES <= 113 * 1024 && TMEM_COLS <= 256) ? 2 : 1;
 };
 
-template <int D, int KV>
-__global__ void __launch_bounds__(ATT_THREADS, AttnCfg<D, KV>::MIN_CTAS)
+template <int D>
+__global__ void __launch_bounds__(ATT_THREADS, AttnCfg<D>::MIN_CTAS)
 attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK0,
                  const __grid_constant__ CUtensorMap tmV0, const __grid_constant__ CUtensorMap tmK1,
                  const __grid_constant__ CUtensorMap tmV1, const AttnKParams p) {
-  using Cfg = AttnCfg<D, KV>;
+  using Cfg = AttnCfg<D>;
   constexpr int ND = Cfg::ND, BKV = Cfg::BKV, STAGES = Cfg::STAGES, DV = Cfg::DV;
   extern __shared__ __align__(1024) uint8_t smem[];
   if ((smem_u32(smem) & 1023u) != 0) {  // SWIZZLE_128B tiles need it; no slack is budgeted (see Cfg)
@@ -115,8 +113,6 @@ attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_launch_dependents();  // the next kernel's prologue may overlap this kernel (host.cuh launch_pdl)
-  pdl_wait();               // operands come from earlier kernels: nothing above touched global memory
 
   if (warp == 0) {
     // ===================== TMA producer =====================
@@ -313,19 +309,9 @@ attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
   }
 }
 
-// 4-D view (d, head, token, batch) of an fp16 [batch*rows, ld] matrix whose head h occupies
-// columns [h*d, (h+1)*d) from `base`.
-static int make_head_tmap(CUtensorMap* m, const void* base, int d, int heads, int rows, int batch,
-                          int ld, int box_rows) {
-  const uint64_t dims[4] = {(uint64_t)d, (uint64_t)heads, (uint64_t)rows, (uint64_t)batch};
-  const uint64_t strides[3] = {(uint64_t)d * 2, (uint64_t)ld * 2, (uint64_t)rows * ld * 2};
-  const uint32_t box[4] = {64u, 1u, (uint32_t)box_rows, 1u};
-  return encode_tmap_f16(m, base, 4, dims, strides, box);
-}
-
-template <int D, int KV>
+template <int D>
 static int launch_attention(const idiff_attn_args* a, cudaStream_t stream) {
-  using Cfg = AttnCfg<D, KV>;
+  using Cfg = AttnCfg<D>;
   CUtensorMap tmQ, tmK0, tmV0, tmK1, tmV1;
   if (make_head_tmap(&tmQ, a->q, D, a->heads, a->nq, a->batch, a->q_ld, BQ)) return -1;
   if (make_head_tmap(&tmK0, a->k0, D, a->heads, a->n0, a->batch, a->k0_ld, Cfg::BKV)) return -1;
@@ -349,13 +335,13 @@ static int launch_attention(const idiff_attn_args* a, cudaStream_t stream) {
   p.out_ld = a->out_ld;
   static bool attr_set = false;
   if (!attr_set) {
-    IDIFF_CHECK_CUDA(cudaFuncSetAttribute(attention_kernel<D, KV>,
+    IDIFF_CHECK_CUDA(cudaFuncSetAttribute(attention_kernel<D>,
                                           cudaFuncAttributeMaxDynamicSharedMemorySize,
                                           Cfg::SMEM_BYTES));
     attr_set = true;
   }
   dim3 grid((a->nq + BQ - 1) / BQ, a->heads, a->batch);
-  IDIFF_CHECK_CUDA(launch_pdl(attention_kernel<D, KV>, dim3(grid), dim3(ATT_THREADS), Cfg::SMEM_BYTES, stream, tmQ, tmK0, tmV0, tmK1, tmV1, p));
+  attention_kernel<D><<<grid, ATT_THREADS, Cfg::SMEM_BYTES, stream>>>(tmQ, tmK0, tmV0, tmK1, tmV1, p);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -380,23 +366,9 @@ extern "C" int idiff_attention(const idiff_attn_args* a, void* stream) {
     return att2::attention_v2_d40(a, s);
   }
   switch (a->head_dim) {
-    case 40: {
-      // attention2.cu (two Q tiles, f16x2 exponentials, tensor-core row sums) is the production
-      // kernel for d=40; IDIFF_ATTN_V1=1 selects the first-generation kernel for A/B runs.
-      static const bool use_v1 = []() {
-        const char* e = getenv("IDIFF_ATTN_V1");
-        return e && e[0] == '1';
-      }();
-      return use_v1 ? launch_attention<40, 128>(a, s) : att2::attention_v2_d40(a, s);
-    }
-    case 80: {
-      static const bool wide = []() {
-        const char* e = getenv("IDIFF_ATT_BKV");
-        return e && atoi(e) == 128;
-      }();
-      return wide ? launch_attention<80, 128>(a, s) : launch_attention<80, 64>(a, s);
-    }
-    case 160: return launch_attention<160, 64>(a, s);
+    case 40: return att2::attention_v2_d40(a, s);  // attention2.cu: two Q tiles per CTA, FMA-pipe exponentials
+    case 80: return launch_attention<80>(a, s);
+    case 160: return launch_attention<160>(a, s);
     default: return set_error("idiff_attention: unsupported head_dim %d (40/80/160)", a->head_dim);
   }
 }

@@ -216,7 +216,6 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
     if (TRACE && traced) trace_buf[slot] = clock();
   };
 
-  pdl_launch_dependents();  // the next kernel's prologue may overlap this kernel (host.cuh launch_pdl)
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int q0 = blockIdx.x * 2 * BQ;
@@ -249,7 +248,6 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();  // Q / K / V come from the previous kernel: nothing above touched global memory
 
   // Register re-partition between warpgroups (the setmaxnreg must sit at the head of each role
   // branch so that ptxas allocates the branch bodies against the new limits).
@@ -554,14 +552,6 @@ attention2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
   }
 }
 
-static int make_head_tmap(CUtensorMap* m, const void* base, int d, int heads, int rows, int batch,
-                          int ld, int box_rows) {
-  const uint64_t dims[4] = {(uint64_t)d, (uint64_t)heads, (uint64_t)rows, (uint64_t)batch};
-  const uint64_t strides[3] = {(uint64_t)d * 2, (uint64_t)ld * 2, (uint64_t)rows * ld * 2};
-  const uint32_t box[4] = {64u, 1u, (uint32_t)box_rows, 1u};
-  return encode_tmap_f16(m, base, 4, dims, strides, box);
-}
-
 int attention_v2_d40(const idiff_attn_args* a, cudaStream_t stream) {
   constexpr int D = 40;
   using C = Cfg<D>;
@@ -589,29 +579,21 @@ int attention_v2_d40(const idiff_attn_args* a, cudaStream_t stream) {
   p.mask_q = reinterpret_cast<const uint32_t*>(a->mask_q);
   p.mask_k = reinterpret_cast<const uint32_t*>(a->mask_k);
   static const bool trace = getenv("IDIFF_ATT2_TRACE") != nullptr;
-  // share of the exponentials taken on the FMA pipe: pairs per 8 (IDIFF_ATT2_POLY=0..4, tuning knob)
-  static const int poly = []() {
-    const char* e = getenv("IDIFF_ATT2_POLY");
-    const int v = e ? atoi(e) : 2;  // measured (B200, batch 8, 4096 keys): 0: 420, 2: 408, 3: 430, 4: 456 us
-    return (v >= 0 && v <= 4) ? v : 2;
-  }();
   const bool masked = a->mask_q != nullptr;
+  // unmasked: pairs 1 and 5 of every 8 score pairs take the FMA-pipe exp2 (measured on a B200, batch 8, 4096 keys:
+  // 408 us, against 420 / 430 / 456 us for 0 / 3 / 4 of 8 pairs)
   auto kern = masked ? attention2_kernel<D, false, 0u, true>
               : trace ? attention2_kernel<D, true, 0u>
-              : poly == 0 ? attention2_kernel<D, false, 0u>
-              : poly == 1 ? attention2_kernel<D, false, 0x10u>
-              : poly == 2 ? attention2_kernel<D, false, 0x22u>
-              : poly == 3 ? attention2_kernel<D, false, 0x4Au>
-                          : attention2_kernel<D, false, 0xAAu>;
+                      : attention2_kernel<D, false, 0x22u>;
   const int smem_bytes = C::SMEM_BYTES + (trace ? C::TRACE_BYTES : 0);
-  static bool attr_set[2] = {false, false};  // (per masked / unmasked kernel; the env knobs are read once)
+  static bool attr_set[2] = {false, false};  // (per masked / unmasked kernel; IDIFF_ATT2_TRACE is read once)
   if (!attr_set[masked]) {
     IDIFF_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
     IDIFF_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
     attr_set[masked] = true;
   }
   dim3 grid((a->nq + 2 * BQ - 1) / (2 * BQ), a->heads, a->batch);
-  IDIFF_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(THREADS), smem_bytes, stream, tmQ, tmK0, tmV0, tmK1, tmV1, p));
+  kern<<<grid, THREADS, smem_bytes, stream>>>(tmQ, tmK0, tmV0, tmK1, tmV1, p);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

@@ -19,8 +19,6 @@ namespace idiff {
 __global__ void __launch_bounds__(128)
 embed_tokens_kernel(const long long* __restrict__ ids, const uint4* __restrict__ tok, const uint4* __restrict__ pos,
                     uint4* __restrict__ out, int rows, int T, int vocab, int CV) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int row = blockIdx.x;
   if (row >= rows) return;
   long long id = ids[row];
@@ -48,8 +46,6 @@ __global__ void __launch_bounds__(128)
 causal_attention_small_kernel(const h16* __restrict__ q, const h16* __restrict__ k, const h16* __restrict__ v,
                               h16* __restrict__ out, const int* __restrict__ key_len, int ld, int ld_out, int T,
                               float scale_log2e) {
-  pdl_launch_dependents();
-  pdl_wait();
   extern __shared__ float cas_smem[];
   float* sK = cas_smem;                 // [T][D]
   float* sV = cas_smem + (size_t)T * D;  // [T][D]
@@ -127,9 +123,9 @@ extern "C" int idiff_embed_tokens(const long long* ids, const void* tok_table, c
   IDIFF_REQUIRE(rows > 0 && tokens_per_seq > 0 && vocab > 0 && channels > 0 && channels % 8 == 0 && rows % tokens_per_seq == 0,
                 "idiff_embed_tokens: bad shape rows=%d tokens=%d vocab=%d C=%d (C %% 8 == 0, rows %% tokens == 0)", rows,
                 tokens_per_seq, vocab, channels);
-  IDIFF_CHECK_CUDA(launch_pdl(embed_tokens_kernel, dim3(rows), dim3(128), 0, reinterpret_cast<cudaStream_t>(stream), ids,
-                              reinterpret_cast<const uint4*>(tok_table), reinterpret_cast<const uint4*>(pos_table),
-                              reinterpret_cast<uint4*>(out), rows, tokens_per_seq, vocab, channels / 8));
+  embed_tokens_kernel<<<rows, 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(ids,
+      reinterpret_cast<const uint4*>(tok_table), reinterpret_cast<const uint4*>(pos_table),
+      reinterpret_cast<uint4*>(out), rows, tokens_per_seq, vocab, channels / 8);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -153,10 +149,9 @@ extern "C" int idiff_causal_attention_small(const void* q, const void* k, const 
                                           2 * 128 * 64 * (int)sizeof(float)));
     attr_set = true;
   }
-  IDIFF_CHECK_CUDA(launch_pdl(causal_attention_small_kernel<64>, dim3(heads, batch), dim3(128), smem,
-                              reinterpret_cast<cudaStream_t>(stream), reinterpret_cast<const h16*>(q),
-                              reinterpret_cast<const h16*>(k), reinterpret_cast<const h16*>(v), reinterpret_cast<h16*>(out),
-                              key_len, ld_qkv, ld_out, tokens, scale * 1.4426950408889634f));
+  causal_attention_small_kernel<64><<<dim3(heads, batch), 128, smem, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const h16*>(q),
+      reinterpret_cast<const h16*>(k), reinterpret_cast<const h16*>(v), reinterpret_cast<h16*>(out), key_len, ld_qkv,
+      ld_out, tokens, scale * 1.4426950408889634f);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

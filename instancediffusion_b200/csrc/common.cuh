@@ -24,13 +24,6 @@ namespace idiff {
 
 #define IDIFF_DEVICE __device__ __forceinline__
 
-// Programmatic dependent launch (host.cuh launch_pdl): launch_dependents lets the next kernel in the
-// stream become resident and run its prologue while this one is still working; wait blocks until the
-// previous kernel has completed and its global writes are visible.  Both are no-ops for a kernel
-// launched without the attribute.
-IDIFF_DEVICE void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;\n" ::: "memory"); }
-IDIFF_DEVICE void pdl_wait() { asm volatile("griddepcontrol.wait;\n" ::: "memory"); }
-
 IDIFF_DEVICE uint32_t smem_u32(const void* p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }
@@ -169,61 +162,6 @@ IDIFF_DEVICE void tmem_dealloc(uint32_t taddr) {  // whole warp
   asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;\n" ::"r"(taddr), "n"(kCols)
                : "memory");
 }
-// ---- cta_group::2 (a CTA pair = one TPC shares each UMMA; both CTAs take part in alloc / dealloc) ----
-template <uint32_t kCols>
-IDIFF_DEVICE void tmem_alloc_cg2(uint32_t* smem_dst) {  // whole warp, in BOTH CTAs of the pair
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;\n" ::"r"(smem_u32(smem_dst)), "n"(kCols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;\n" ::: "memory");
-}
-template <uint32_t kCols>
-IDIFF_DEVICE void tmem_dealloc_cg2(uint32_t taddr) {  // whole warp, in both CTAs, after a cluster barrier
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;\n" ::"r"(taddr), "n"(kCols) : "memory");
-}
-// arrive (once all previously issued UMMAs of this thread have completed) on the mbarrier at this shared-memory
-// offset in BOTH CTAs of the pair
-IDIFF_DEVICE void umma_commit_cg2(uint64_t* bar) {
-  const uint16_t mask = 3;
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;\n" ::"r"(
-          smem_u32(bar)),
-      "h"(mask)
-      : "memory");
-}
-IDIFF_DEVICE void cluster_sync() {  // all threads of all CTAs of the cluster
-  asm volatile("barrier.cluster.arrive.release.aligned;\n" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;\n" ::: "memory");
-}
-// arrive on the mbarrier at the same shared-memory offset in CTA `rank` of the cluster
-IDIFF_DEVICE void mbar_arrive_remote(uint64_t* bar, uint32_t rank) {
-  uint32_t raddr;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;\n" : "=r"(raddr) : "r"(smem_u32(bar)), "r"(rank));
-  // default semantics (.release.cta) as in CUTLASS' ClusterBarrier::arrive(cta_id): an explicit .release.cluster
-  // costs a cluster-scope fence per arrive (~1 us each: measured, the whole pipeline ran at one k-block per us)
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];\n" ::"r"(raddr) : "memory");
-}
-// bounded wait on a local mbarrier whose arrivals come from the peer CTA
-IDIFF_DEVICE void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  const long long t0 = clock64();
-  uint32_t spins = 0;
-  for (;;) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}\n"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    if (ok) return;
-    if ((++spins & 0x3ff) == 0 && (clock64() - t0) > 8000000000LL) {
-      printf("idiff: cluster mbarrier timeout block=(%d,%d,%d) thread=%d bar=%u parity=%u\n", blockIdx.x, blockIdx.y,
-             blockIdx.z, threadIdx.x, smem_u32(bar), parity);
-      __trap();
-    }
-  }
-}
-
 IDIFF_DEVICE void tc_fence_before() {
   asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory");
 }

@@ -25,8 +25,6 @@ __global__ void __launch_bounds__(256)
 segs_inconv_kernel(const float* __restrict__ segs, const float* __restrict__ w, const float* __restrict__ bias,
                    h16* __restrict__ y, float* __restrict__ seg_sum, int B, int CI, int S, int R,
                    long sb, long sc, long sy, long sx) {
-  pdl_launch_dependents();
-  pdl_wait();
   __shared__ float sw[3 * INCONV_MAX_CI * 9];
   __shared__ float red[8];
   for (int i = threadIdx.x; i < 3 * CI * 9; i += blockDim.x) sw[i] = w[i];
@@ -91,8 +89,6 @@ segs_inconv_kernel(const float* __restrict__ segs, const float* __restrict__ w, 
 template <int VEC>
 __global__ void patchify_kernel(const h16* __restrict__ x, h16* __restrict__ y, int B, int H, int W, int C,
                                 int p) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int CV = C / VEC;
   const int Ho = H / p, Wo = W / p;
   const long total = (long)B * Ho * Wo * p * p * CV;
@@ -121,8 +117,6 @@ __global__ void patchify_kernel(const h16* __restrict__ x, h16* __restrict__ y, 
 __global__ void __launch_bounds__(256)
 dwconv7x7_kernel(const uint4* __restrict__ x, const float* __restrict__ w, const float* __restrict__ bias,
                  uint4* __restrict__ y, int B, int H, int W, int C) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int CV = C >> 3;
   const long total = (long)B * H * W * CV;
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
@@ -173,8 +167,6 @@ dwconv7x7_kernel(const uint4* __restrict__ x, const float* __restrict__ w, const
 __global__ void seg_tokens_kernel(const h16* __restrict__ feat, const h16* __restrict__ null_pos,
                                   const float* __restrict__ pos, const float* __restrict__ seg_sum,
                                   h16* __restrict__ out, int B, int P, int C, int T) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int F = C * P / T;
   const long total = (long)B * T * F;
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
@@ -211,8 +203,8 @@ extern "C" int idiff_segs_inconv(const float* segs, const long* strides, const f
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   IDIFF_CHECK_CUDA(cudaMemsetAsync(seg_sum, 0, sizeof(float) * batch, s));
   dim3 grid((out_size + 255) / 256, out_size, batch);
-  IDIFF_CHECK_CUDA(launch_pdl(segs_inconv_kernel, grid, dim3(256), 0, s, segs, w, bias, reinterpret_cast<h16*>(y),
-                              seg_sum, batch, cin, in_size, out_size, strides[0], strides[1], strides[2], strides[3]));
+  segs_inconv_kernel<<<grid, 256, 0, s>>>(segs, w, bias, reinterpret_cast<h16*>(y), seg_sum, batch, cin, in_size,
+                                          out_size, strides[0], strides[1], strides[2], strides[3]);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -226,10 +218,10 @@ extern "C" int idiff_patchify(const void* x, void* y, int batch, int h, int w, i
   h16* yo = reinterpret_cast<h16*>(y);
   if (c % 8 == 0) {
     const long total = (long)batch * h * w * (c / 8);
-    IDIFF_CHECK_CUDA(launch_pdl(patchify_kernel<8>, dim3(grid_for(total, 256)), dim3(256), 0, s, xi, yo, batch, h, w, c, p));
+    patchify_kernel<8><<<grid_for(total, 256), 256, 0, s>>>(xi, yo, batch, h, w, c, p);
   } else {
     const long total = (long)batch * h * w * c;
-    IDIFF_CHECK_CUDA(launch_pdl(patchify_kernel<1>, dim3(grid_for(total, 256)), dim3(256), 0, s, xi, yo, batch, h, w, c, p));
+    patchify_kernel<1><<<grid_for(total, 256), 256, 0, s>>>(xi, yo, batch, h, w, c, p);
   }
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
@@ -242,8 +234,8 @@ extern "C" int idiff_dwconv7x7(const void* x, const float* w, const float* bias,
   IDIFF_REQUIRE(c % 8 == 0, "idiff_dwconv7x7: C=%d must be a multiple of 8", c);
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   const long total = (long)batch * h * w_ * (c / 8);
-  IDIFF_CHECK_CUDA(launch_pdl(dwconv7x7_kernel, dim3(grid_for(total, 256)), dim3(256), 0, s,
-                              reinterpret_cast<const uint4*>(x), w, bias, reinterpret_cast<uint4*>(y), batch, h, w_, c));
+  dwconv7x7_kernel<<<grid_for(total, 256), 256, 0, s>>>(reinterpret_cast<const uint4*>(x), w, bias,
+                                                        reinterpret_cast<uint4*>(y), batch, h, w_, c);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -256,9 +248,9 @@ extern "C" int idiff_seg_tokens(const void* feat, const void* null_pos, const fl
                 "idiff_seg_tokens: C*P=%ld must be a multiple of the token count %d", (long)channels * pixels, tokens);
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   const long total = (long)batch * channels * pixels;
-  IDIFF_CHECK_CUDA(launch_pdl(seg_tokens_kernel, dim3(grid_for(total, 256)), dim3(256), 0, s,
-                              reinterpret_cast<const h16*>(feat), reinterpret_cast<const h16*>(null_pos), pos,
-                              seg_sum, reinterpret_cast<h16*>(out), batch, pixels, channels, tokens));
+  seg_tokens_kernel<<<grid_for(total, 256), 256, 0, s>>>(reinterpret_cast<const h16*>(feat),
+                                                         reinterpret_cast<const h16*>(null_pos), pos, seg_sum,
+                                                         reinterpret_cast<h16*>(out), batch, pixels, channels, tokens);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

@@ -13,8 +13,6 @@ namespace idiff {
 // ---------------------------------------------------------------------------------------------
 __global__ void nchw_f32_to_nhwc_f16_kernel(const float* __restrict__ x, h16* __restrict__ y, int B,
                                             int C, int HW, int CP) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   const long total = (long)B * HW * CP;
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
     const int c = (int)(i % CP);
@@ -26,8 +24,6 @@ __global__ void nchw_f32_to_nhwc_f16_kernel(const float* __restrict__ x, h16* __
 }
 __global__ void nhwc_f16_to_nchw_f32_kernel(const h16* __restrict__ x, float* __restrict__ y, int B,
                                             int C, int HW) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   __shared__ float tile[32][33];
   // grid: (HW/32, C/32, B)
   const int b = blockIdx.z;
@@ -46,8 +42,6 @@ __global__ void nhwc_f16_to_nchw_f32_kernel(const h16* __restrict__ x, float* __
 // F.interpolate(scale_factor=2, mode="nearest") (openaimodel.py:107), NHWC, 8 channels/thread
 __global__ void upsample2x_kernel(const uint4* __restrict__ x, uint4* __restrict__ y, int B, int H, int W,
                                   int CV) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   const long total = (long)B * 4 * H * W * CV;
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
     const int cv = (int)(i % CV);
@@ -65,8 +59,6 @@ __global__ void upsample2x_kernel(const uint4* __restrict__ x, uint4* __restrict
 // asymmetric F.pad (0,1,0,1) + stride-2 padding-0 convolution (diffusionmodules/model.py:70-74)
 __global__ void im2col_s2_kernel(const uint4* __restrict__ x, uint4* __restrict__ y, int B, int H, int W,
                                  int CV, int pad_lo) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   const int Ho = H >> 1, Wo = W >> 1;
   const long total = (long)B * Ho * Wo * 9 * CV;
   const uint4 zero = make_uint4(0, 0, 0, 0);
@@ -95,8 +87,6 @@ fourier_embed_kernel(const float* __restrict__ coords, const float* __restrict__
                      const float* __restrict__ text, const float* __restrict__ null_text,
                      const float* __restrict__ null_pos, h16* __restrict__ out, int D,
                      int text_dim, int out_ld, int mask_mode, int dropped) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   __shared__ float red[8];
   __shared__ float s_mpos;
   const int row = blockIdx.x;
@@ -142,8 +132,6 @@ fourier_embed_kernel(const float* __restrict__ coords, const float* __restrict__
 // timestep_embedding (util.py:160-180): [cos(t f) | sin(t f)], f_k = exp(-ln(1e4) k / half)
 __global__ void timestep_embedding_kernel(const float* __restrict__ t, h16* __restrict__ out, int B,
                                           int dim) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   const int half_dim = dim >> 1;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * half_dim) return;
@@ -163,8 +151,6 @@ __global__ void plms_update_kernel(const float* __restrict__ x, const float* __r
                                    float c1, float c2, float c3, float sqrt_at, float sqrt_aprev,
                                    float sqrt_1m_at, float sqrt_1m_aprev, float* __restrict__ e_out,
                                    float* __restrict__ x_out, long n) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) {
     float e = e_c[i];
     if (e_u) {
@@ -184,8 +170,6 @@ __global__ void plms_update_kernel(const float* __restrict__ x, const float* __r
 
 __global__ void latent_mean_kernel(const float* const* __restrict__ xs, int count, float* __restrict__ out,
                                    long n) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) {
     float s = 0.f;
     for (int k = 0; k < count; ++k) s += xs[k][i];
@@ -194,8 +178,6 @@ __global__ void latent_mean_kernel(const float* const* __restrict__ xs, int coun
 }
 
 __global__ void silu_f16_kernel(const h16* __restrict__ x, h16* __restrict__ y, long n) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x)
     y[i] = f2h(silu_f(h2f(x[i])));
 }
@@ -213,8 +195,6 @@ static inline int grid_for(long total, int threads) {
 // one thread per (b, k, a, c) element of att_masks
 __global__ void boxes_to_attmask_kernel(const float* __restrict__ boxes, const int* __restrict__ counts,
                                         float* __restrict__ att, int B, int K, int S) {
-  pdl_launch_dependents();
-  pdl_wait();
   const long total = (long)B * K * S * S;
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
     const int c = (int)(i % S);
@@ -238,8 +218,6 @@ __global__ void boxes_to_attmask_kernel(const float* __restrict__ boxes, const i
 // one thread per (b, token): token < P visual, then 4*K object tokens, then `tail`
 __global__ void attmask_words_kernel(const float* __restrict__ att, const int* __restrict__ active,
                                      uint32_t* __restrict__ mq, uint32_t* __restrict__ mk, int B, int K, int P, int tail) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int NK = P + 4 * K + tail;
   const long total = (long)B * NK;
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
@@ -272,7 +250,8 @@ extern "C" int idiff_nchw_f32_to_nhwc_f16(const float* x, void* y, int batch, in
                                           void* stream) {
   IDIFF_REQUIRE(x && y && c_pad >= c, "idiff_nchw_f32_to_nhwc_f16: bad arguments");
   const long total = (long)batch * hw * c_pad;
-  IDIFF_CHECK_CUDA(launch_pdl(nchw_f32_to_nhwc_f16_kernel, dim3(grid_for(total, 256)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream),  x, reinterpret_cast<h16*>(y), batch, c, hw, c_pad));
+  nchw_f32_to_nhwc_f16_kernel<<<grid_for(total, 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(x,
+      reinterpret_cast<h16*>(y), batch, c, hw, c_pad);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -280,7 +259,8 @@ extern "C" int idiff_nchw_f32_to_nhwc_f16(const float* x, void* y, int batch, in
 extern "C" int idiff_nhwc_f16_to_nchw_f32(const void* x, float* y, int batch, int c, int hw, void* stream) {
   IDIFF_REQUIRE(x && y, "idiff_nhwc_f16_to_nchw_f32: null pointer argument");
   dim3 grid((hw + 31) / 32, (c + 31) / 32, batch);
-  IDIFF_CHECK_CUDA(launch_pdl(nhwc_f16_to_nchw_f32_kernel, dim3(grid), dim3(dim3(32, 8)), 0, reinterpret_cast<cudaStream_t>(stream),  reinterpret_cast<const h16*>(x), y, batch, c, hw));
+  nhwc_f16_to_nchw_f32_kernel<<<grid, dim3(32, 8), 0, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const h16*>(x),
+      y, batch, c, hw);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -288,7 +268,8 @@ extern "C" int idiff_nhwc_f16_to_nchw_f32(const void* x, float* y, int batch, in
 extern "C" int idiff_upsample_nearest2x(const void* x, void* y, int batch, int h, int w, int c, void* stream) {
   IDIFF_REQUIRE(x && y && c % 8 == 0, "idiff_upsample_nearest2x: bad arguments");
   const long total = (long)batch * 4 * h * w * (c / 8);
-  IDIFF_CHECK_CUDA(launch_pdl(upsample2x_kernel, dim3(grid_for(total, 256)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream),  reinterpret_cast<const uint4*>(x), reinterpret_cast<uint4*>(y), batch, h, w, c / 8));
+  upsample2x_kernel<<<grid_for(total, 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const uint4*>(x),
+      reinterpret_cast<uint4*>(y), batch, h, w, c / 8);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -296,7 +277,8 @@ extern "C" int idiff_upsample_nearest2x(const void* x, void* y, int batch, int h
 extern "C" int idiff_im2col_s2(const void* x, void* y, int batch, int h, int w, int c, void* stream) {
   IDIFF_REQUIRE(x && y && c % 8 == 0 && h % 2 == 0 && w % 2 == 0, "idiff_im2col_s2: bad arguments");
   const long total = (long)batch * (h / 2) * (w / 2) * 9 * (c / 8);
-  IDIFF_CHECK_CUDA(launch_pdl(im2col_s2_kernel, dim3(grid_for(total, 256)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream),  reinterpret_cast<const uint4*>(x), reinterpret_cast<uint4*>(y), batch, h, w, c / 8, 1));
+  im2col_s2_kernel<<<grid_for(total, 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const uint4*>(x),
+      reinterpret_cast<uint4*>(y), batch, h, w, c / 8, 1);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -304,7 +286,8 @@ extern "C" int idiff_im2col_s2(const void* x, void* y, int batch, int h, int w, 
 extern "C" int idiff_im2col_s2_pad01(const void* x, void* y, int batch, int h, int w, int c, void* stream) {
   IDIFF_REQUIRE(x && y && c % 8 == 0 && h % 2 == 0 && w % 2 == 0, "idiff_im2col_s2_pad01: bad arguments");
   const long total = (long)batch * (h / 2) * (w / 2) * 9 * (c / 8);
-  IDIFF_CHECK_CUDA(launch_pdl(im2col_s2_kernel, dim3(grid_for(total, 256)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream),  reinterpret_cast<const uint4*>(x), reinterpret_cast<uint4*>(y), batch, h, w, c / 8, 0));
+  im2col_s2_kernel<<<grid_for(total, 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const uint4*>(x),
+      reinterpret_cast<uint4*>(y), batch, h, w, c / 8, 0);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -322,7 +305,8 @@ extern "C" int idiff_fourier_embed(const float* coords, const float* masks, cons
     IDIFF_CHECK_CUDA(cudaMemcpyToSymbol(c_freqs, f, sizeof(f)));
     freqs_set = true;
   }
-  IDIFF_CHECK_CUDA(launch_pdl(fourier_embed_kernel, dim3(rows), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream),  coords, masks, text, null_text, null_pos, reinterpret_cast<h16*>(out), coord_dim, text ? text_dim : 0, out_ld, mask_mode, dropped));
+  fourier_embed_kernel<<<rows, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(coords, masks, text, null_text,
+      null_pos, reinterpret_cast<h16*>(out), coord_dim, text ? text_dim : 0, out_ld, mask_mode, dropped);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -330,7 +314,8 @@ extern "C" int idiff_fourier_embed(const float* coords, const float* masks, cons
 extern "C" int idiff_timestep_embedding(const float* t, void* out, int batch, int dim, void* stream) {
   IDIFF_REQUIRE(t && out && dim % 2 == 0, "idiff_timestep_embedding: bad arguments");
   const int total = batch * dim / 2;
-  IDIFF_CHECK_CUDA(launch_pdl(timestep_embedding_kernel, dim3((total + 127) / 128), dim3(128), 0, reinterpret_cast<cudaStream_t>(stream),  t, reinterpret_cast<h16*>(out), batch, dim));
+  timestep_embedding_kernel<<<(total + 127) / 128, 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(t,
+      reinterpret_cast<h16*>(out), batch, dim);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -340,21 +325,23 @@ extern "C" int idiff_plms_update(const float* x, const float* e_c, const float* 
                                  float c1, float c2, float c3, float a_t, float a_prev,
                                  float sqrt_one_minus_at, float* e_out, float* x_out, long n, void* stream) {
   IDIFF_REQUIRE(x && e_c && x_out && n > 0, "idiff_plms_update: bad arguments");
-  IDIFF_CHECK_CUDA(launch_pdl(plms_update_kernel, dim3(grid_for(n, 256)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream),  x, e_c, e_u, gs, old1, old2, old3, c0, c1, c2, c3, sqrtf(a_t), sqrtf(a_prev), sqrt_one_minus_at, sqrtf(1.0f - a_prev), e_out, x_out, n));
+  plms_update_kernel<<<grid_for(n, 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(x, e_c, e_u, gs, old1, old2,
+      old3, c0, c1, c2, c3, sqrtf(a_t), sqrtf(a_prev), sqrt_one_minus_at, sqrtf(1.0f - a_prev), e_out, x_out, n);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
 
 extern "C" int idiff_latent_mean(const float* const* xs_dev, int count, float* out, long n, void* stream) {
   IDIFF_REQUIRE(xs_dev && out && count > 0, "idiff_latent_mean: bad arguments");
-  IDIFF_CHECK_CUDA(launch_pdl(latent_mean_kernel, dim3(grid_for(n, 256)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream), xs_dev, count, out, n));
+  latent_mean_kernel<<<grid_for(n, 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(xs_dev, count, out, n);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
 
 extern "C" int idiff_silu_f16(const void* x, void* y, long n, void* stream) {
   IDIFF_REQUIRE(x && y && n > 0, "idiff_silu_f16: bad arguments");
-  IDIFF_CHECK_CUDA(launch_pdl(silu_f16_kernel, dim3(grid_for(n, 256)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream),  reinterpret_cast<const h16*>(x), reinterpret_cast<h16*>(y), n));
+  silu_f16_kernel<<<grid_for(n, 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const h16*>(x),
+      reinterpret_cast<h16*>(y), n);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -364,8 +351,8 @@ extern "C" int idiff_boxes_to_attmask(const float* boxes, const int* counts, flo
   using namespace idiff;
   IDIFF_REQUIRE(boxes && counts && att_masks && batch > 0 && max_objs > 0 && size > 0, "idiff_boxes_to_attmask: bad arguments");
   const long total = (long)batch * max_objs * size * size;
-  IDIFF_CHECK_CUDA(launch_pdl(boxes_to_attmask_kernel, dim3(grid_for(total, 256)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream),
-                              boxes, counts, att_masks, batch, max_objs, size));
+  boxes_to_attmask_kernel<<<grid_for(total, 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(boxes, counts,
+      att_masks, batch, max_objs, size);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -376,9 +363,8 @@ extern "C" int idiff_attmask_words(const float* att_masks, const int* active, vo
   IDIFF_REQUIRE(att_masks && active && mask_q && mask_k, "idiff_attmask_words: null pointer argument");
   IDIFF_REQUIRE(n_objs > 0 && n_objs <= 30 && pixels > 0 && tail >= 0, "idiff_attmask_words: 1..30 instances supported (got %d)", n_objs);
   const long total = (long)batch * (pixels + 4 * n_objs + tail);
-  IDIFF_CHECK_CUDA(launch_pdl(attmask_words_kernel, dim3(grid_for(total, 256)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream),
-                              att_masks, active, reinterpret_cast<uint32_t*>(mask_q), reinterpret_cast<uint32_t*>(mask_k), batch,
-                              n_objs, pixels, tail));
+  attmask_words_kernel<<<grid_for(total, 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(att_masks, active,
+      reinterpret_cast<uint32_t*>(mask_q), reinterpret_cast<uint32_t*>(mask_k), batch, n_objs, pixels, tail);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

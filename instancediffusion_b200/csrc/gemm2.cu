@@ -37,12 +37,10 @@ namespace v2 {
 constexpr int BM = 128;
 constexpr int BK = 64;
 constexpr int A_STAGE_BYTES = BM * BK * 2;
-// Warpgroup 0 = {TMA, UMMA, 2 idle warps}; then EW epilogue warps (EW / 4 per TMEM lane quarter).
-// Only EW = 8 (two column halves, 224 registers per epilogue warp) is instantiated: EW = 12 and 16 (three /
-// four column parts, 152 / 104 registers) were built and measured slower for every shape of this UNet -- the
-// TMEM read path and, at 16, register spills cost more than the extra warps hide (profiles/README.md round 2).
-// The kernel keeps EW as a template parameter; the register split for the other values is left in place.
-constexpr int MAX_EPI_WARPS = 16;
+// Warpgroup 0 = {TMA, UMMA, 2 idle warps}; then EW epilogue warps (EW / 4 per TMEM lane quarter: two column
+// halves, 224 registers per epilogue warp).  12 / 16 epilogue warps and CTA pairs (cta_group::2) were measured
+// slower or no faster: profiles/README.md round 2, sections 7.3 and 7.5.
+constexpr int EW = 8;
 constexpr int CHUNK = 16;  // accumulator columns per tcgen05.ld
 constexpr int EPI_TAB_PB = 4;  // batches a conv tile may straddle and still use the smem epilogue table
 
@@ -61,7 +59,7 @@ struct Params {
   float gate;
   // stream-K fixup
   float* ws;    // [G][BN/CHUNK][128][CHUNK] fp32 partial tiles
-  int* sflags;  // [G][EPI_WARPS] publish flags (fixed location, self-resetting)
+  int* sflags;  // [G][EW] publish flags (fixed location, self-resetting)
   unsigned long long* trace;  // optional [G][8] %globaltimer stamps (idiff_set_gemm_trace), else null
   // LayerNorm folded across GEMMs (header: ln_* fields)
   float2* ln_out;        // producer: [n_tiles * PARTS][M] partial (sum, sumsq) of the output rows
@@ -76,14 +74,13 @@ struct Params {
 // 16-byte global access per thread and row (which costs an L1 transaction per access: measured
 // ~0.7 us per chunk, tools/trace_gemm.py).  The staging buffer takes smem from the operand ring,
 // so it is used for the short-K layers (epilogue-bound); long-K convolutions keep the deep ring.
-template <int BN, bool TMA_EPI, int EW = 8, int CG = 1>
+template <int BN, bool TMA_EPI>
 struct Cfg {
-  static_assert(CG == 1 || CG == 2, "cta_group 1 or 2");
   static constexpr int THREADS = 128 + EW * 32;
   static constexpr int PARTS = EW / 4;            // column parts of a tile (one epilogue warp per quarter and part)
   static constexpr int NCHT = BN / CHUNK;         // 16-column accumulator chunks of a tile
   static constexpr int NCH_MAX = (NCHT + PARTS - 1) / PARTS;  // ... owned by one warp, at most
-  static constexpr int B_STAGE_BYTES = (BN / CG) * BK * 2;  // cta_group::2: each CTA of the pair stages half of B
+  static constexpr int B_STAGE_BYTES = BN * BK * 2;
   static constexpr int STAGE_BYTES = A_STAGE_BYTES + B_STAGE_BYTES;
   static constexpr int BOX_BYTES = 32 * CHUNK * 2;                       // 1 KiB
   // TMA epilogue staging: one [32 rows x BN/2 columns] fp16 box per epilogue warp (row-major, no swizzle):
@@ -91,7 +88,7 @@ struct Cfg {
   static constexpr int WBOX_BYTES = 32 * (BN / 2) * 2;
   static constexpr int STG_BYTES = TMA_EPI ? EW * WBOX_BYTES : 0;
   static constexpr int TAB_BYTES = 2 * EPI_TAB_PB * BN * 4;
-  static constexpr int BAR_BYTES = 1024;  // 2*STAGES + 4 + MAX_EPI_WARPS mbarriers (<= 32 x 8 B) + the TMEM base slot;
+  static constexpr int BAR_BYTES = 1024;  // 2*STAGES + 4 + EW mbarriers + the TMEM base slot;
                                           // 1 KiB keeps the staging boxes 1024-byte aligned (SWIZZLE_128B boxes)
   static constexpr int FIXED = 1024 + BAR_BYTES + TAB_BYTES + STG_BYTES;
   static constexpr int STAGES_FIT = (227 * 1024 - FIXED) / STAGE_BYTES;
@@ -355,20 +352,13 @@ constexpr int MODE_PLAIN = 0;  // bias / row-add table, optional SiLU, optional 
 constexpr int MODE_GEGLU = 1;  // (value + b) * gelu(gate + b), fp16 out with N/2 columns
 constexpr int MODE_NCHW = 2;   // fp32 (B, N, HW) output (the final conv -> eps)
 
-// CG = 2: the kernel runs as clusters of two CTAs (one TPC) that share each UMMA: tcgen05.mma.cta_group::2 with
-// M = 256 -- every CTA stages its own 128 A rows and HALF of the B tile, the tensor cores of both SMs read both
-// halves.  Measured (tools/r2_probe2.py, profiles/README.md round 2): the 1-CTA SS-mode UMMA is bound by its
-// shared-memory operand fetch at ~64 B/clk (128 x 256 x 16: 12 KB = 192 clk against 128 clk of math; 128 x 160:
-// 9 KB = 144 against 80), not by issue, TMA or L2; halving B per SM brings 256-wide tiles to the math rate.
-// The leader CTA (cluster rank 0) issues; the peer forwards its "operands landed" barrier phases.
-template <int BN, int MODE, bool TMA_EPI, int EW, int CG = 1, bool REALLOC = true>
+template <int BN, int MODE, bool TMA_EPI>
 __global__ void __launch_bounds__(128 + EW * 32, 1)
 gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
              const __grid_constant__ CUtensorMap tmO, const __grid_constant__ CUtensorMap tmR,
              const Params p) {
-  using C = Cfg<BN, TMA_EPI, EW, CG>;
+  using C = Cfg<BN, TMA_EPI>;
   constexpr int STAGES = C::STAGES;
-  constexpr int EPI_WARPS = EW;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
                                              ~static_cast<uintptr_t>(1023));
@@ -379,17 +369,14 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
   uint64_t* empty_bar = bars + STAGES;
   uint64_t* tmem_full = bars + 2 * STAGES;       // [2]
   uint64_t* tmem_empty = bars + 2 * STAGES + 2;  // [2]
-  uint64_t* res_bar = bars + 2 * STAGES + 4;     // [EPI_WARPS] residual boxes landed (TMA_EPI)
-  uint64_t* peer_full = bars + 2 * STAGES + 4 + MAX_EPI_WARPS;  // [STAGES] (CG 2, leader): the peer's operands landed
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3 * STAGES + 4 + MAX_EPI_WARPS);
+  uint64_t* res_bar = bars + 2 * STAGES + 4;     // [EW] residual boxes landed (TMA_EPI)
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 4 + EW);
   float* s_epi = reinterpret_cast<float*>(smem + STAGES * C::STAGE_BYTES + C::BAR_BYTES);  // [2][EPI_TAB_PB][BN]
   uint8_t* s_stage = smem + STAGES * C::STAGE_BYTES + C::BAR_BYTES + C::TAB_BYTES;          // [quarter][NCHT][1 KiB]
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  uint32_t crank = 0;  // rank in the CTA pair
-  if constexpr (CG == 2) asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(crank));
-  const int cta = (CG == 2) ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;  // index in the work schedule (pair / CTA)
+  const int cta = blockIdx.x;
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
@@ -400,27 +387,20 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
     }
     for (int a = 0; a < 2; ++a) {
       mbar_init(&tmem_full[a], 1);
-      mbar_init(&tmem_empty[a], CG * EPI_WARPS * 32);  // (CG 2: the leader's barrier also counts the peer's epilogue)
+      mbar_init(&tmem_empty[a], EW * 32);
     }
-    for (int s = 0; s < STAGES; ++s) mbar_init(&peer_full[s], 1);
-    for (int w = 0; w < EPI_WARPS; ++w) mbar_init(&res_bar[w], 1);
+    for (int w = 0; w < EW; ++w) mbar_init(&res_bar[w], 1);
     if (TMA_EPI) {
       tma_prefetch_desc(&tmO);
       tma_prefetch_desc(&tmR);
     }
     fence_barrier_init();
   }
-  if (warp == 1) {
-    if constexpr (CG == 2) tmem_alloc_cg2<C::TMEM_COLS>(tmem_slot);  // collective over the pair: same columns in both SMs
-    else tmem_alloc<C::TMEM_COLS>(tmem_slot);
-  }
+  if (warp == 1) tmem_alloc<C::TMEM_COLS>(tmem_slot);
   tc_fence_before();
-  if constexpr (CG == 2) cluster_sync();  // barriers of BOTH CTAs are initialised before any remote arrive / commit
-  else __syncthreads();
+  __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_launch_dependents();  // the next kernel's prologue may overlap this kernel (host.cuh launch_pdl)
-  pdl_wait();               // operands come from earlier kernels: nothing above touched global memory
   auto stamp = [&](int slot) {
     if (p.trace) {
       unsigned long long t;
@@ -435,7 +415,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
 
   auto tile_origin = [&](int tile, int& n0, int& m0, int& b0, int& h0, int& w0) {
     const int n_tile = tile % p.n_tiles;
-    const int m_tile = (CG == 2) ? 2 * (tile / p.n_tiles) + (int)crank : tile / p.n_tiles;  // pair tile = 2 stacked M tiles
+    const int m_tile = tile / p.n_tiles;
     n0 = n_tile * BN;
     m0 = m_tile * BM;
     b0 = h0 = w0 = 0;
@@ -452,11 +432,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
   // Warpgroup 0 = {TMA, UMMA, 2 idle warps} gives registers to the two epilogue warpgroups
   // (setmaxnreg at the head of each role branch: 56*128 + 224*256 = the CTA's 168*384 allocation).
   if (warp < 4) {
-  // launch allocation -> after the split:  EW 8: 384 x 168 = 128 x 56 + 256 x 224;  EW 12: 512 x 128 = 128 x 56 +
-  // 384 x 152;  EW 16: 640 x 96 >= 128 x 48 + 512 x 104
-  if constexpr (!REALLOC) {  // diagnostic variant: every warp keeps its launch allocation
-  } else if constexpr (EW == 16) asm volatile("setmaxnreg.dec.sync.aligned.u32 48;\n");
-  else asm volatile("setmaxnreg.dec.sync.aligned.u32 56;\n");
+  asm volatile("setmaxnreg.dec.sync.aligned.u32 56;\n");
   if (warp == 0) {
     // ===================== TMA producer =====================
     if (lane == 0) {
@@ -467,7 +443,6 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
       while (it.next(sg)) {
         int n0, m0, b0, h0, w0;
         tile_origin(sg.tile, n0, m0, b0, h0, w0);
-        const int nb = n0 + (int)crank * (BN / CG) * (CG - 1);  // CG 2: this CTA's half of the B tile
         // conv: k-block kb = (tap, 64-channel slice cb); walked incrementally
         int tap = 0, cb = 0, ky = 0, kx = 0;
         if (p.conv) {
@@ -491,7 +466,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
           } else {
             tma_load_2d(sA + s * A_STAGE_BYTES, &tmA, &full_bar[s], kb * BK, m0);
           }
-          tma_load_2d(sB + s * C::B_STAGE_BYTES, &tmB, &full_bar[s], kb * BK, nb);
+          tma_load_2d(sB + s * C::B_STAGE_BYTES, &tmB, &full_bar[s], kb * BK, n0);
           if (++s == STAGES) {
             s = 0;
             ph ^= 1;
@@ -506,95 +481,56 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
     // per UMMA; this way they live in uniform registers and the four UMMAs of a k-block issue back to back
     // (UTCHMMA x4, UTCBAR).  Descriptors = (low word + constant high word), one add per UMMA; running
     // stage / phase instead of div / mod.
-    constexpr uint32_t idesc = make_idesc_f16(BM * CG, BN, UMMA_AB_FMT, 0, 0);
+    constexpr uint32_t idesc = make_idesc_f16(BM, BN, UMMA_AB_FMT, 0, 0);
     constexpr uint32_t DESC_HI = (1024u >> 4) | (1u << 14) | (2u << 29);  // SBO 1024 B, version 1, SWIZZLE_128B
     const uint32_t a_lo0 = ((smem_u32(sA) & 0x3FFFFu) >> 4) | (1u << 16);  // LBO (unused, swizzled K-major) = 16 B
     const uint32_t b_lo0 = ((smem_u32(sB) & 0x3FFFFu) >> 4) | (1u << 16);
     auto umma_lo = [&](uint32_t d_tmem, uint32_t a_lo, uint32_t b_lo, uint32_t acc) {
-      if constexpr (CG == 2) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-            "mov.b64 da, {%1, %3};\n\t"
-            "mov.b64 db, {%2, %3};\n\t"
-            "setp.ne.b32 p, %5, 0;\n\t"
-            "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %4, p;\n\t}\n" ::"r"(d_tmem),
-            "r"(a_lo), "r"(b_lo), "r"(DESC_HI), "r"(idesc), "r"(acc)
-            : "memory");
-      } else {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-            "mov.b64 da, {%1, %3};\n\t"
-            "mov.b64 db, {%2, %3};\n\t"
-            "setp.ne.b32 p, %5, 0;\n\t"
-            "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %4, p;\n\t}\n" ::"r"(d_tmem),
-            "r"(a_lo), "r"(b_lo), "r"(DESC_HI), "r"(idesc), "r"(acc)
-            : "memory");
-      }
+      asm volatile(
+          "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
+          "mov.b64 da, {%1, %3};\n\t"
+          "mov.b64 db, {%2, %3};\n\t"
+          "setp.ne.b32 p, %5, 0;\n\t"
+          "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %4, p;\n\t}\n" ::"r"(d_tmem),
+          "r"(a_lo), "r"(b_lo), "r"(DESC_HI), "r"(idesc), "r"(acc)
+          : "memory");
     };
-    auto commit = [&](uint64_t* bar) {  // CG 2: the arrival lands on the barrier at this offset in BOTH CTAs
-      if constexpr (CG == 2) umma_commit_cg2(bar);
-      else umma_commit(bar);
-    };
-    if (CG == 1 || crank == 0) {
-      WorkIter it(p, cta);
-      Seg sg;
-      uint32_t sc = 0, s = 0, ph = 0;
-      bool first = true;
-      while (it.next(sg)) {
-        const int acc = sc & 1;
-        if constexpr (CG == 2) mbar_wait_cluster(&tmem_empty[acc], ((sc >> 1) & 1) ^ 1);
-        else mbar_wait(&tmem_empty[acc], ((sc >> 1) & 1) ^ 1);
+    WorkIter it(p, cta);
+    Seg sg;
+    uint32_t sc = 0, s = 0, ph = 0;
+    bool first = true;
+    while (it.next(sg)) {
+      const int acc = sc & 1;
+      mbar_wait(&tmem_empty[acc], ((sc >> 1) & 1) ^ 1);
+      tc_fence_after();
+      const uint32_t d_tmem = tmem_base + acc * C::ACC_STRIDE;
+      for (int kb = sg.kb0; kb < sg.kb1; ++kb) {
+        mbar_wait(&full_bar[s], ph);
+        if (first && lane == 0) stamp(1);
+        first = false;
         tc_fence_after();
-        const uint32_t d_tmem = tmem_base + acc * C::ACC_STRIDE;
-        for (int kb = sg.kb0; kb < sg.kb1; ++kb) {
-          mbar_wait(&full_bar[s], ph);
-          if constexpr (CG == 2) mbar_wait_cluster(&peer_full[s], ph);
-          if (first && lane == 0) stamp(1);
-          first = false;
-          tc_fence_after();
-          const uint32_t a_lo = a_lo0 + s * (A_STAGE_BYTES >> 4);
-          const uint32_t b_lo = b_lo0 + s * (C::B_STAGE_BYTES >> 4);
-          if (elect_one()) {
+        const uint32_t a_lo = a_lo0 + s * (A_STAGE_BYTES >> 4);
+        const uint32_t b_lo = b_lo0 + s * (C::B_STAGE_BYTES >> 4);
+        if (elect_one()) {
 #pragma unroll
-            for (int k = 0; k < BK / 16; ++k) umma_lo(d_tmem, a_lo + 2 * k, b_lo + 2 * k, (kb > sg.kb0 || k > 0) ? 1u : 0u);
-            commit(&empty_bar[s]);
-          }
-          __syncwarp();
-          if (++s == STAGES) {
-            s = 0;
-            ph ^= 1;
-          }
+          for (int k = 0; k < BK / 16; ++k) umma_lo(d_tmem, a_lo + 2 * k, b_lo + 2 * k, (kb > sg.kb0 || k > 0) ? 1u : 0u);
+          umma_commit(&empty_bar[s]);
         }
-        if (elect_one()) commit(&tmem_full[acc]);
         __syncwarp();
-        if (sc == 0 && lane == 0) stamp(2);
-        ++sc;
-      }
-    } else {
-      // CG 2, peer CTA: tell the leader when this CTA's operands of each stage have landed
-      if (lane == 0) {
-        WorkIter it(p, cta);
-        Seg sg;
-        uint32_t s = 0, ph = 0;
-        while (it.next(sg)) {
-          for (int kb = sg.kb0; kb < sg.kb1; ++kb) {
-            mbar_wait(&full_bar[s], ph);
-            mbar_arrive_remote(&peer_full[s], 0);
-            if (++s == STAGES) {
-              s = 0;
-              ph ^= 1;
-            }
-          }
+        if (++s == STAGES) {
+          s = 0;
+          ph ^= 1;
         }
       }
+      if (elect_one()) umma_commit(&tmem_full[acc]);
+      __syncwarp();
+      if (sc == 0 && lane == 0) stamp(2);
+      ++sc;
     }
     __syncwarp();
   }
   } else {
-    if constexpr (!REALLOC) {
-    } else if constexpr (EW == 8) asm volatile("setmaxnreg.inc.sync.aligned.u32 224;\n");
-    else if constexpr (EW == 12) asm volatile("setmaxnreg.inc.sync.aligned.u32 152;\n");
-    else asm volatile("setmaxnreg.inc.sync.aligned.u32 104;\n");
+    asm volatile("setmaxnreg.inc.sync.aligned.u32 224;\n");
     // ===================== epilogue (warps 4..11) =====================
     const int ew = warp - 4;       // 0..7
     const int quarter = warp & 3;  // TMEM lane quarter this warp may access
@@ -713,7 +649,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
       if (owner) {
         const int npb = tab_rowadd ? p.PB : 1;
         const int et = threadIdx.x - 128;  // 0..255
-        for (int idx = et; idx < npb * BN; idx += EPI_WARPS * 32) {
+        for (int idx = et; idx < npb * BN; idx += EW * 32) {
           const int pb = idx / BN, c = idx - pb * BN;
           const int col = n0 + c;
           float val = 0.f;
@@ -724,7 +660,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
           tab[idx] = val;
           if (p.ln_in) tab[BN + idx] = (col < p.N) ? __ldg(p.ln_s + col) : 0.f;  // row 1: sum_k W'[col, k]
         }
-        asm volatile("bar.sync 1, %0;\n" ::"n"(EPI_WARPS * 32) : "memory");
+        asm volatile("bar.sync 1, %0;\n" ::"n"(EW * 32) : "memory");
       }
       const float* tab_row = tab + ((tab_rowadd && p.conv) ? (r / (p.PW * p.PH)) * BN : 0);
       // LayerNorm fold, consumer side: this row's mean / rstd from the producer GEMM's partial sums, added
@@ -769,16 +705,16 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
                                         __uint_as_float(v[4 * q + 2]), __uint_as_float(v[4 * q + 3])));
         }
         tc_fence_before();
-        mbar_arrive(&tmem_empty[acc]);  // (stream-K is never scheduled for CTA pairs)
+        mbar_arrive(&tmem_empty[acc]);
         // __syncwarp orders the lanes' partial stores before lane 0's release store (cumulative), so a
         // single release replaces 32 per-thread __threadfence() (MEMBAR.GPU + L1 invalidate each).
         __syncwarp();
-        if (lane == 0) st_release_gpu(p.sflags + cta * EPI_WARPS + ew, 1);
+        if (lane == 0) st_release_gpu(p.sflags + cta * EW + ew, 1);
       } else {
         // ---- owner: (optional fixup) + fused epilogue ----
         if (fixup) {
           for (int f = f0; f <= f1; ++f) {
-            const int* fl = p.sflags + f * EPI_WARPS + ew;
+            const int* fl = p.sflags + f * EW + ew;
             const long long t0 = clock64();
             while (ld_acquire_gpu(fl) == 0) {
               if (clock64() - t0 > 8000000000LL) {
@@ -1007,7 +943,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
         // before one wait, all results are staged before one proxy fence / warp sync, and the
         // group's TMA stores go out together.  (Chunk-at-a-time was a ~1200-cycle serial dependency
         // chain per 16 columns with only two warps per scheduler to hide it: tools/trace_gemm.py.)
-        constexpr int GROUP = (EW == 16) ? 2 : 4;  // 104-register epilogue warps hold two chunks at a time
+        constexpr int GROUP = 4;
         constexpr int NV = (NOUT_CH + PARTS - 1) / PARTS;  // output chunks of this warp, at most
 #pragma unroll
         for (int g0 = 0; g0 < NV; g0 += GROUP) {
@@ -1180,13 +1116,12 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
           __stcg(p.ln_out + (long)((sg.tile % p.n_tiles) * PARTS + part) * p.M + out_row, make_float2(ln_ps, ln_pq));
         if (sc == 0 && threadIdx.x == 128) stamp(5);
         tc_fence_before();
-        if (CG == 2 && crank != 0) mbar_arrive_remote(&tmem_empty[acc], 0);  // the leader's issuer waits for both epilogues
-        else mbar_arrive(&tmem_empty[acc]);
+        mbar_arrive(&tmem_empty[acc]);
         if (fixup) {
           // consume the followers' flags so the next launch (or graph replay) starts clean
           __syncwarp();
           if (lane == 0)
-            for (int f = f0; f <= f1; ++f) st_release_gpu(p.sflags + f * EPI_WARPS + ew, 0);
+            for (int f = f0; f <= f1; ++f) st_release_gpu(p.sflags + f * EW + ew, 0);
         }
       }
       ++sc;
@@ -1195,20 +1130,14 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
 
   if (TMA_EPI && warp >= 4 && lane == 0) tma_store_wait_read();  // boxes must outlive their stores
   if (threadIdx.x == 128) stamp(6);
-  if constexpr (CG == 2) {
-    tc_fence_before();
-    cluster_sync();  // no CTA of the pair leaves (or frees tensor memory) while the other may still signal / read it
-  } else {
-    __syncthreads();
-  }
+  __syncthreads();
   if (threadIdx.x == 0) {
     stamp(7);
     if (p.trace) p.trace[(long)blockIdx.x * 16 + 13] = (unsigned long long)clock64();  // SM clock at exit
   }
   if (warp == 1) {
     tc_fence_after();
-    if constexpr (CG == 2) tmem_dealloc_cg2<C::TMEM_COLS>(tmem_base);
-    else tmem_dealloc<C::TMEM_COLS>(tmem_base);
+    tmem_dealloc<C::TMEM_COLS>(tmem_base);
   }
 }
 
@@ -1220,10 +1149,8 @@ static unsigned long long* g_trace = nullptr;
 static long g_ws_bytes = 0;
 static int g_num_sms = 0;
 constexpr long kFlagBytes = 64 * 1024;
-static int kTmaEpiMaxKB = []() {
-  const char* e = getenv("IDIFF_TMA_EPI_MAX_KB");  // tuning knob: k-blocks up to which the TMA epilogue is used
-  return e ? atoi(e) : 40;
-}();
+// k-blocks up to which the TMA epilogue is used; the LayerNorm fold (ln_stats_in) exists only in that epilogue
+constexpr int kTmaEpiMaxKB = 40;
 
 static void choose_patch(int H, int W, int* PW, int* PH, int* PB) {
   int pw = 1;
@@ -1235,10 +1162,9 @@ static void choose_patch(int H, int W, int* PW, int* PH, int* PB) {
   *PB = 128 / (pw * ph);
 }
 
-template <int BN, int MODE, bool TMA_EPI, int CG = 1>
+template <int BN, int MODE, bool TMA_EPI>
 static int launch(const idiff_gemm_args* a, cudaStream_t stream, bool want_sk) {
-  constexpr int EW = 8;
-  using C = Cfg<BN, TMA_EPI, EW, CG>;
+  using C = Cfg<BN, TMA_EPI>;
   Params p;
   memset(&p, 0, sizeof(p));
   p.M = a->M;
@@ -1294,11 +1220,11 @@ static int launch(const idiff_gemm_args* a, cudaStream_t stream, bool want_sk) {
   {
     const uint64_t dims[2] = {(uint64_t)a->K, (uint64_t)a->N};
     const uint64_t strides[1] = {(uint64_t)a->ldw * 2};
-    const uint32_t box[2] = {(uint32_t)BK, (uint32_t)(BN / CG)};  // CG 2: each CTA of the pair loads half of the N tile
+    const uint32_t box[2] = {(uint32_t)BK, (uint32_t)BN};
     if (encode_tmap_f16(&tmB, a->w, 2, dims, strides, box)) return -1;
   }
   p.n_tiles = (a->N + BN - 1) / BN;
-  p.T = p.n_tiles * ((m_tiles + CG - 1) / CG);  // CG 2: a work item is a pair of stacked M tiles
+  p.T = p.n_tiles * m_tiles;
 
   if (g_num_sms == 0) {
     int dev = 0;
@@ -1312,8 +1238,7 @@ static int launch(const idiff_gemm_args* a, cudaStream_t stream, bool want_sk) {
   // takes precedence over the process-wide default of idiff_set_gemm_workspace
   void* ws_ptr = a->workspace ? a->workspace : g_ws;
   const long ws_bytes = a->workspace ? a->workspace_bytes : g_ws_bytes;
-  const int workers = g_num_sms / CG;  // CTAs, or CTA pairs (one per TPC)
-  const bool use_sk = CG == 1 && want_sk && ws_ptr && ws_bytes >= ws_need && p.KB >= 8 && (p.T % g_num_sms) != 0 &&
+  const bool use_sk = want_sk && ws_ptr && ws_bytes >= ws_need && p.KB >= 8 && (p.T % g_num_sms) != 0 &&
                       (long)p.T * p.KB >= g_num_sms;
   if (use_sk) {
     p.G = g_num_sms;
@@ -1323,7 +1248,7 @@ static int launch(const idiff_gemm_args* a, cudaStream_t stream, bool want_sk) {
     p.sflags = reinterpret_cast<int*>(ws_ptr);
     p.ws = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(ws_ptr) + kFlagBytes);
   } else {
-    p.G = workers < p.T ? workers : p.T;
+    p.G = g_num_sms < p.T ? g_num_sms : p.T;
     p.T_dp = p.T;
     p.U_sk = 0;
   }
@@ -1353,12 +1278,11 @@ static int launch(const idiff_gemm_args* a, cudaStream_t stream, bool want_sk) {
 
   static bool attr_set = false;
   if (!attr_set) {
-    IDIFF_CHECK_CUDA(cudaFuncSetAttribute(gemm2_kernel<BN, MODE, TMA_EPI, EW, CG>,
+    IDIFF_CHECK_CUDA(cudaFuncSetAttribute(gemm2_kernel<BN, MODE, TMA_EPI>,
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
     attr_set = true;
   }
-  IDIFF_CHECK_CUDA(launch_pdl_cluster(gemm2_kernel<BN, MODE, TMA_EPI, EW, CG>, dim3(p.G * CG), dim3(C::THREADS), C::SMEM_BYTES,
-                                      stream, CG, tmA, tmB, tmO, tmR, p));
+  gemm2_kernel<BN, MODE, TMA_EPI><<<p.G, C::THREADS, C::SMEM_BYTES, stream>>>(tmA, tmB, tmO, tmR, p);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -1446,62 +1370,41 @@ static Plan plan_gemm(const idiff_gemm_args* a, int fixed_bn) {  // fixed_bn: 0 
 }
 
 struct Resolved {
-  int bn, mode, ew, cg;
+  int bn, mode;
   bool tma_epi, sk;
 };
-
-// CTA pairs (cta_group::2) or single CTAs?  Measured on the B200 (tools/bench_kernels.py, profiles/README.md round 2):
-// the pair kernel is correct at every shape (IDIFF_GEMM_CG=2 runs the whole kernel suite) and its k-block is ~11 %
-// cheaper (conv 320->320 @64: 917 vs 1035 clk), but it runs plain rounds of 256-row work items over 74 TPCs without
-// stream-K and loses that again to tile quantisation (84 vs 82 us); tools/micro/umma_bench2.cu shows why the k-block
-// does not reach the 4 x N/2 clk of math in either mode: the two-barrier operand ring has a ~2700 clk turnaround
-// (commit -> empty barrier -> producer -> full barrier -> issuer), which six 36 KB stages of N = 160 do not cover.
-// Single CTAs stay the default; IDIFF_GEMM_CG=2 selects pairs for every eligible GEMM (A/B runs).
-static int choose_cg(const idiff_gemm_args* a, int bn, bool sk1) {
-  (void)a; (void)bn; (void)sk1;
-  static const int forced = []() {
-    const char* e = getenv("IDIFF_GEMM_CG");
-    return e ? atoi(e) : 0;
-  }();
-  return forced == 2 ? 2 : 1;
-}
 
 static Resolved resolve(const idiff_gemm_args* a) {
   Resolved r;
   // GEGLU: one 256-column accumulator tile = 128 value columns + their 128 gates (packing.py)
   if (a->flags & IDIFF_EPI_GEGLU) {
     const bool sk = plan_gemm(a, 256).sk;
-    r = {256, MODE_GEGLU, 8, choose_cg(a, 256, sk), true, sk};
+    r = {256, MODE_GEGLU, true, sk};
     return r;
   }
   if (a->flags & IDIFF_OUT_F32_NCHW) {
-    r = {128, MODE_NCHW, 8, 1, false, plan_gemm(a, 128).sk};
+    r = {128, MODE_NCHW, false, plan_gemm(a, 128).sk};
     return r;
   }
   // short K: the epilogue dominates -> TMA-staged epilogue (shallower operand ring);
   // long K (3x3 convolutions): deep operand ring, direct epilogue hidden behind the next mainloop
   const bool tma_epi = ((a->K + BK - 1) / BK) <= kTmaEpiMaxKB;
   const Plan pl = plan_gemm(a, false);
-  r = {pl.bn, MODE_PLAIN, 8, choose_cg(a, pl.bn, pl.sk), tma_epi, pl.sk};
+  r = {pl.bn, MODE_PLAIN, tma_epi, pl.sk};
   return r;
 }
 
 template <int BN>
 static int launch_plain(const Resolved& r, const idiff_gemm_args* a, cudaStream_t stream) {
-  if (r.cg == 2) return r.tma_epi ? launch<BN, MODE_PLAIN, true, 2>(a, stream, false) : launch<BN, MODE_PLAIN, false, 2>(a, stream, false);
-  return r.tma_epi ? launch<BN, MODE_PLAIN, true, 1>(a, stream, r.sk) : launch<BN, MODE_PLAIN, false, 1>(a, stream, r.sk);
+  return r.tma_epi ? launch<BN, MODE_PLAIN, true>(a, stream, r.sk) : launch<BN, MODE_PLAIN, false>(a, stream, r.sk);
 }
 
-// One instantiation per (tile width, epilogue mode, cta_group): each kernel carries only its own mode's code (an
+// One instantiation per (tile width, epilogue mode, TMA epilogue): each kernel carries only its own mode's code (an
 // all-modes kernel was ~140 KB of SASS and stalled on instruction fetch: 26 % stall_no_inst, profiles/).
-// The epilogue-warp count is a template parameter of the kernel; 12 and 16 warps (three / four column parts,
-// 152 / 104 registers) were measured SLOWER than 8 at every UNet shape (profiles/README.md, round 2: qkv C320
-// 41 -> 45 -> 66 us) and are not instantiated.
 int gemm_v2(const idiff_gemm_args* a, cudaStream_t stream) {
   const Resolved r = resolve(a);
-  if (r.mode == MODE_GEGLU)
-    return r.cg == 2 ? launch<256, MODE_GEGLU, true, 2>(a, stream, false) : launch<256, MODE_GEGLU, true, 1>(a, stream, r.sk);
-  if (r.mode == MODE_NCHW) return launch<128, MODE_NCHW, false, 1>(a, stream, r.sk);
+  if (r.mode == MODE_GEGLU) return launch<256, MODE_GEGLU, true>(a, stream, r.sk);
+  if (r.mode == MODE_NCHW) return launch<128, MODE_NCHW, false>(a, stream, r.sk);
   switch (r.bn) {
     case 256: return launch_plain<256>(r, a, stream);
     case 192: return launch_plain<192>(r, a, stream);
@@ -1513,7 +1416,7 @@ int gemm_v2(const idiff_gemm_args* a, cudaStream_t stream) {
 // slots of the LayerNorm partial statistics a producer GEMM with these arguments writes per row
 int ln_slots_of(const idiff_gemm_args* a) {
   const Resolved r = resolve(a);
-  return ((a->N + r.bn - 1) / r.bn) * (r.ew / 4);
+  return ((a->N + r.bn - 1) / r.bn) * (EW / 4);  // (n tile, column part): Cfg::PARTS
 }
 
 }  // namespace v2
@@ -1546,7 +1449,8 @@ extern "C" int idiff_gemm(const idiff_gemm_args* a, void* stream) {
   if (a->ln_stats_in) {
     IDIFF_REQUIRE(a->ln_colsum && a->ln_slots_in > 0 && a->ln_slots_in <= 64, "idiff_gemm: LayerNorm fold needs ln_colsum and 1..64 slots");
     IDIFF_REQUIRE(a->conv_h == 0 && !nchw && !a->rowadd, "idiff_gemm: LayerNorm fold applies to plain / GEGLU linear layers");
-    IDIFF_REQUIRE((a->K + 63) / 64 <= 40, "idiff_gemm: LayerNorm fold needs K <= 2560 (K=%d)", a->K);
+    IDIFF_REQUIRE((a->K + v2::BK - 1) / v2::BK <= v2::kTmaEpiMaxKB, "idiff_gemm: LayerNorm fold needs K <= %d (K=%d)",
+                  v2::BK * v2::kTmaEpiMaxKB, a->K);
     IDIFF_REQUIRE((reinterpret_cast<uintptr_t>(a->ln_stats_in) & 7) == 0, "idiff_gemm: ln_stats_in must be 8B aligned");
   }
   if (a->ln_stats_out) {

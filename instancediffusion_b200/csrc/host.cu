@@ -1,7 +1,6 @@
 // Error text + TMA descriptor encoding (driver entry point resolved at run time, so the
 // library links against cudart only and loads on a GPU-less box).
 #include "host.cuh"
-#include <stdlib.h>
 
 #include <mutex>
 #include <string.h>
@@ -77,12 +76,11 @@ int encode_tmap_f16_sw(CUtensorMap* map, const void* base, int rank, const uint6
   return 0;
 }
 
-bool pdl_enabled() {
-  static const bool on = []() {
-    const char* e = getenv("IDIFF_PDL");
-    return e && e[0] == '1';  // opt-in: measured neutral on the UNet forward (17.44 vs 17.43 ms)
-  }();
-  return on;
+int make_head_tmap(CUtensorMap* m, const void* base, int d, int heads, int rows, int batch, int ld, int box_rows) {
+  const uint64_t dims[4] = {(uint64_t)d, (uint64_t)heads, (uint64_t)rows, (uint64_t)batch};
+  const uint64_t strides[3] = {(uint64_t)d * 2, (uint64_t)ld * 2, (uint64_t)rows * ld * 2};
+  const uint32_t box[4] = {64u, 1u, (uint32_t)box_rows, 1u};
+  return encode_tmap_f16(m, base, 4, dims, strides, box);
 }
 
 }  // namespace idiff

@@ -35,56 +35,8 @@ int encode_tmap_f16(CUtensorMap* map, const void* base, int rank, const uint64_t
 int encode_tmap_f16_sw(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
                        const uint64_t* strides_bytes, const uint32_t* box, int swizzle_bytes);
 
-// Launch with programmatic stream serialization ("programmatic dependent launch"): the kernel may
-// become resident while its predecessor in the stream is still running; every kernel of this library
-// calls pdl_wait() (common.cuh) before it touches global memory, so only launch latency and prologues
-// (barrier init, TMEM allocation, descriptor prefetch) overlap.  About 500 dependent launches make one
-// UNet forward.  Opt-in with IDIFF_PDL=1: measured neutral inside the CUDA graph (the big kernels fill
-// the register file, so a successor cannot become resident before they exit); plain stream order is
-// the default.
-bool pdl_enabled();
-template <typename... KArgs, typename... Args>
-cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                       Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
-// same, launched as thread-block clusters of `cluster_x` CTAs along x (1 = no cluster attribute)
-template <typename... KArgs, typename... Args>
-cudaError_t launch_pdl_cluster(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                               int cluster_x, Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  int n = 0;
-  if (cluster_x > 1) {
-    attr[n].id = cudaLaunchAttributeClusterDimension;
-    attr[n].val.clusterDim.x = cluster_x;
-    attr[n].val.clusterDim.y = 1;
-    attr[n].val.clusterDim.z = 1;
-    ++n;
-  }
-  if (pdl_enabled()) {
-    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n].val.programmaticStreamSerializationAllowed = 1;
-    ++n;
-  }
-  cfg.attrs = attr;
-  cfg.numAttrs = n;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
+// 4-D view (d, head, token, batch) of a 16-bit [batch*rows, ld] matrix whose head h occupies
+// columns [h*d, (h+1)*d) from `base`; boxes of 64 d x 1 head x box_rows tokens (the attention kernels).
+int make_head_tmap(CUtensorMap* m, const void* base, int d, int heads, int rows, int batch, int ld, int box_rows);
 
 }  // namespace idiff

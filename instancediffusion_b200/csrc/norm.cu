@@ -35,8 +35,6 @@ IDIFF_DEVICE void unpack8(const uint4& v, float (&f)[8]) {
 __global__ void __launch_bounds__(512)
 gn_stats_kernel(const uint4* __restrict__ x, float* __restrict__ partial, int hw, int C, int groups,
                 int pix_per_block, int k) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   extern __shared__ float red[];  // [k][C][2]
   const int CV = C >> 3;
   const int r = threadIdx.x / CV;
@@ -126,8 +124,6 @@ __global__ void __launch_bounds__(512)
 gn_apply_kernel(const uint4* __restrict__ x, uint4* __restrict__ y, const float* __restrict__ gamma,
                 const float* __restrict__ beta, const float* __restrict__ partial, int hw, int C,
                 int groups, float eps, int fuse_silu, int pix_per_block, int k, int stat_chunks) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   __shared__ float s_mean[GN_MAX_GROUPS], s_rstd[GN_MAX_GROUPS];
   const int CV = C >> 3;
   const int b = blockIdx.y;
@@ -242,8 +238,6 @@ __global__ void __launch_bounds__(512)
 gn_fused_kernel(const uint4* __restrict__ x, uint4* __restrict__ y, const float* __restrict__ gamma,
                 const float* __restrict__ beta, int hw, int C, int groups, float eps, int fuse_silu, int CS,
                 int CL, int k) {
-  pdl_launch_dependents();
-  pdl_wait();
   extern __shared__ __align__(16) uint8_t gnf_smem[];
   __shared__ float cta_part[GNF_MAX_SLAB_GROUPS * 2];  // this CTA's (sum, sumsq) per group of the slab
   __shared__ float s_mean[GNF_MAX_SLAB_GROUPS], s_rstd[GNF_MAX_SLAB_GROUPS];
@@ -368,8 +362,6 @@ template <int LPR>
 __global__ void __launch_bounds__(256)
 layernorm40_kernel(const uint4* __restrict__ x, uint4* __restrict__ y, const float* __restrict__ gamma,
                    const float* __restrict__ beta, int rows, float eps) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   constexpr int C = 40 * LPR;
   constexpr int CV = C / 8;  // 5 * LPR
   constexpr int RPW = 32 / LPR;
@@ -435,8 +427,6 @@ constexpr int LN_MAX_VEC = 5;  // generic path: C <= 1280
 __global__ void __launch_bounds__(256)
 layernorm_generic_kernel(const uint4* __restrict__ x, uint4* __restrict__ y, const float* __restrict__ gamma,
                          const float* __restrict__ beta, int rows, int C, float eps) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (row >= rows) return;
@@ -496,8 +486,6 @@ layernorm_generic_kernel(const uint4* __restrict__ x, uint4* __restrict__ y, con
 // (module-level entry points); inside the UNet the producing GEMM's epilogue writes the statistics.
 __global__ void __launch_bounds__(256)
 row_stats_kernel(const uint4* __restrict__ x, float2* __restrict__ stats, int rows, int CV) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (row >= rows) return;
@@ -526,8 +514,8 @@ extern "C" int idiff_row_stats(const void* x, void* stats, int rows, int channel
   IDIFF_REQUIRE(x && stats && rows > 0, "idiff_row_stats: bad arguments");
   IDIFF_REQUIRE(channels % 8 == 0 && channels > 0, "idiff_row_stats: C=%d must be a multiple of 8", channels);
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  IDIFF_CHECK_CUDA(launch_pdl(row_stats_kernel, dim3((rows + 7) / 8), dim3(256), 0, s, reinterpret_cast<const uint4*>(x),
-                              reinterpret_cast<float2*>(stats), rows, channels / 8));
+  row_stats_kernel<<<(rows + 7) / 8, 256, 0, s>>>(reinterpret_cast<const uint4*>(x), reinterpret_cast<float2*>(stats),
+                                                  rows, channels / 8);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -632,8 +620,10 @@ extern "C" int idiff_groupnorm(const void* x, void* y, const float* gamma, const
   }
   IDIFF_REQUIRE(smem <= 96 * 1024, "idiff_groupnorm: shared memory %zu too large", smem);
   dim3 grid(chunks, batch);
-  IDIFF_CHECK_CUDA(launch_pdl(gn_stats_kernel, dim3(grid), dim3(threads), smem, s, reinterpret_cast<const uint4*>(x), stats_ws, hw, channels, groups, ppb, k));
-  IDIFF_CHECK_CUDA(launch_pdl(gn_apply_kernel, dim3(grid), dim3(threads), 0, s, reinterpret_cast<const uint4*>(x), reinterpret_cast<uint4*>(y), gamma, beta, stats_ws, hw, channels, groups, eps, fuse_silu, ppb, k, chunks));
+  gn_stats_kernel<<<grid, threads, smem, s>>>(reinterpret_cast<const uint4*>(x), stats_ws, hw, channels, groups, ppb, k);
+  IDIFF_CHECK_CUDA(cudaGetLastError());
+  gn_apply_kernel<<<grid, threads, 0, s>>>(reinterpret_cast<const uint4*>(x), reinterpret_cast<uint4*>(y), gamma, beta,
+                                           stats_ws, hw, channels, groups, eps, fuse_silu, ppb, k, chunks);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -657,13 +647,13 @@ extern "C" int idiff_layernorm(const void* x, void* y, const float* gamma, const
     return (rows + rpb - 1) / rpb;
   };
   if (channels == 320) {
-    IDIFF_CHECK_CUDA(launch_pdl(layernorm40_kernel<8>, dim3(blocks(4)), dim3(256), 0, s, xi, yo, gamma, beta, rows, eps));
+    layernorm40_kernel<8><<<blocks(4), 256, 0, s>>>(xi, yo, gamma, beta, rows, eps);
   } else if (channels == 640) {
-    IDIFF_CHECK_CUDA(launch_pdl(layernorm40_kernel<16>, dim3(blocks(2)), dim3(256), 0, s, xi, yo, gamma, beta, rows, eps));
+    layernorm40_kernel<16><<<blocks(2), 256, 0, s>>>(xi, yo, gamma, beta, rows, eps);
   } else if (channels == 1280) {
-    IDIFF_CHECK_CUDA(launch_pdl(layernorm40_kernel<32>, dim3(blocks(1)), dim3(256), 0, s, xi, yo, gamma, beta, rows, eps));
+    layernorm40_kernel<32><<<blocks(1), 256, 0, s>>>(xi, yo, gamma, beta, rows, eps);
   } else {
-    IDIFF_CHECK_CUDA(launch_pdl(layernorm_generic_kernel, dim3(blocks(1)), dim3(256), 0, s, xi, yo, gamma, beta, rows, channels, eps));
+    layernorm_generic_kernel<<<blocks(1), 256, 0, s>>>(xi, yo, gamma, beta, rows, channels, eps);
   }
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;

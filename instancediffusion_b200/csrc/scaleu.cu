@@ -32,8 +32,6 @@ IDIFF_DEVICE void su_unpack8(const uint4& v, float (&f)[8]) {
 __global__ void __launch_bounds__(512)
 scaleu_coef_kernel(const uint4* __restrict__ skip, float* __restrict__ partial, int H, int W, int C,
                    int pix_per_block, int k) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   __shared__ float tab[4 * 128];  // cos tx, sin tx, cos py, sin py
   extern __shared__ float red[];  // [k][C][7]
   float* ctx = tab;
@@ -92,8 +90,6 @@ scaleu_coef_kernel(const uint4* __restrict__ skip, float* __restrict__ partial, 
 // partial [B][chunks][C][8] -> coef [B][C][8], fixed order (one thread per (b, c, q))
 __global__ void __launch_bounds__(256)
 scaleu_reduce_kernel(const float* __restrict__ partial, float* __restrict__ coef, int chunks, int C, int B) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * C * 8) return;
   const int b = i / (C * 8);
@@ -108,8 +104,6 @@ __global__ void __launch_bounds__(512)
 scaleu_apply_kernel(const uint4* __restrict__ h, const uint4* __restrict__ skip, uint4* __restrict__ out,
                     const float* __restrict__ b1, const float* __restrict__ partial, float s_minus_1,
                     int H, int W, int C1, int C2, int pix_per_block, int k, int coef_chunks) {
-  pdl_launch_dependents();  // programmatic dependent launch: the next kernel may start its prologue
-  pdl_wait();               // ... and this one touches global memory only after its predecessor finished
   __shared__ float tab[4 * 128];
   float* ctx = tab;
   float* stx = tab + 128;
@@ -220,12 +214,17 @@ extern "C" int idiff_scaleu_concat(const void* h, const void* skip, void* out, c
     attr_set = true;
   }
   IDIFF_REQUIRE(smem <= 160 * 1024, "idiff_scaleu_concat: shared memory %zu too large", smem);
-  IDIFF_CHECK_CUDA(launch_pdl(scaleu_coef_kernel, dim3(dim3(chunks1, batch)), dim3(k1 * (c2 / 8)), smem, st, reinterpret_cast<const uint4*>(skip), coef_ws, height, width, c2, ppb1, k1));
+  scaleu_coef_kernel<<<dim3(chunks1, batch), k1 * (c2 / 8), smem, st>>>(reinterpret_cast<const uint4*>(skip), coef_ws,
+      height, width, c2, ppb1, k1);
+  IDIFF_CHECK_CUDA(cudaGetLastError());
   float* coef = coef_ws + (long)batch * SU_MAX_CHUNKS * c2 * 8;
-  IDIFF_CHECK_CUDA(launch_pdl(scaleu_reduce_kernel, dim3((batch * c2 * 8 + 255) / 256), dim3(256), 0, st, coef_ws, coef, chunks1, c2, batch));
+  scaleu_reduce_kernel<<<(batch * c2 * 8 + 255) / 256, 256, 0, st>>>(coef_ws, coef, chunks1, c2, batch);
+  IDIFF_CHECK_CUDA(cudaGetLastError());
   int k2, ppb2, chunks2;
   su_geometry(batch, hw, (c1 + c2) / 8, 4096, &k2, &ppb2, &chunks2);
-  IDIFF_CHECK_CUDA(launch_pdl(scaleu_apply_kernel, dim3(dim3(chunks2, batch)), dim3(k2 * ((c1 + c2) / 8)), 0, st,  reinterpret_cast<const uint4*>(h), reinterpret_cast<const uint4*>(skip), reinterpret_cast<uint4*>(out), b1, coef, s - 1.0f, height, width, c1, c2, ppb2, k2, 1));
+  scaleu_apply_kernel<<<dim3(chunks2, batch), k2 * ((c1 + c2) / 8), 0, st>>>(reinterpret_cast<const uint4*>(h),
+      reinterpret_cast<const uint4*>(skip), reinterpret_cast<uint4*>(out), b1, coef, s - 1.0f, height, width, c1, c2,
+      ppb2, k2, 1);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

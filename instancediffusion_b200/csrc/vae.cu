@@ -15,8 +15,6 @@ namespace idiff {
 __global__ void __launch_bounds__(256)
 vae_latent_in_kernel(const float* __restrict__ z, const float* __restrict__ w, const float* __restrict__ bias,
                      float inv_scale, uint4* __restrict__ out, int B, int C, int HW) {
-  pdl_launch_dependents();
-  pdl_wait();
   __shared__ float sw[64], sb[8];
   if (threadIdx.x < C * C) sw[threadIdx.x] = w[threadIdx.x];
   if (threadIdx.x < C) sb[threadIdx.x] = bias[threadIdx.x];
@@ -50,8 +48,6 @@ vae_latent_in_kernel(const float* __restrict__ z, const float* __restrict__ w, c
 // one CTA per row; the row lives in shared memory as fp32 between the passes
 __global__ void __launch_bounds__(256)
 softmax_rows_kernel(h16* __restrict__ x, int n, long ld) {
-  pdl_launch_dependents();
-  pdl_wait();
   extern __shared__ float srow[];
   __shared__ float red[8];
   h16* row = x + (long)blockIdx.x * ld;
@@ -111,8 +107,8 @@ extern "C" int idiff_vae_latent_in(const float* z, const float* w, const float* 
   IDIFF_REQUIRE(channels >= 1 && channels <= 8, "idiff_vae_latent_in: 1..8 latent channels supported (got %d)", channels);
   const long total = (long)batch * hw;
   const int blocks = (int)((total + 255) / 256 < 148 * 8 ? (total + 255) / 256 : 148 * 8);
-  IDIFF_CHECK_CUDA(launch_pdl(vae_latent_in_kernel, dim3(blocks), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream), z, w,
-                              bias, inv_scale, reinterpret_cast<uint4*>(out), batch, channels, hw));
+  vae_latent_in_kernel<<<blocks, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(z, w, bias, inv_scale,
+      reinterpret_cast<uint4*>(out), batch, channels, hw);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -128,8 +124,7 @@ extern "C" int idiff_softmax_rows(void* x, int rows, int n, long ld, void* strea
     IDIFF_CHECK_CUDA(cudaFuncSetAttribute(softmax_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
     attr_set = true;
   }
-  IDIFF_CHECK_CUDA(launch_pdl(softmax_rows_kernel, dim3(rows), dim3(256), smem, reinterpret_cast<cudaStream_t>(stream),
-                              reinterpret_cast<h16*>(x), n, ld));
+  softmax_rows_kernel<<<rows, 256, smem, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<h16*>(x), n, ld);
   IDIFF_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

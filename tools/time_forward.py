@@ -33,4 +33,4 @@ with torch.no_grad():
     torch.cuda.synchronize()
 ms = s.elapsed_time(e) / iters
 tf = 2 * B * (1.136 if alpha else 0.803)
-print(f"forward(batch {2 * B}, alpha={alpha}) {ms:.2f} ms  ~{tf / ms * 1e3:.0f} TFLOP/s (F_min)  v1={os.environ.get('IDIFF_GEMM_V1', '0')}")
+print(f"forward(batch {2 * B}, alpha={alpha}) {ms:.2f} ms  ~{tf / ms * 1e3:.0f} TFLOP/s (F_min)")
